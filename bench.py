@@ -506,6 +506,12 @@ def run_ours(args):
 
     ms_res_1, launches_1, _ = timed_median("resident_one_lane", submit_resident, 1)
     ms_res, launches, per_rank_res = timed_median("resident", submit_resident, L)
+    # what the headline path handed its caller in its last timed step: the map's folded keep mask and that batch's per-node counters
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        n_voi_last, n_flag_last, n_rej_last = lanes[(args.steps - 1) % L].node_stats()
+        outputs = {"map_keep": gmap.get_keep().astype(np.float32), "node_voi_points": n_voi_last.astype(np.float64),
+                   "node_flagged_bins": n_flag_last.astype(np.float64), "node_rejected_points": n_rej_last.astype(np.float64)}
     # --- e2e: host buffers through the same call ---
     ms_e2e_1, _, _ = timed_median("e2e_one_lane", submit_host, 1)
     ms_e2e, _, per_rank_e2e = timed_median("e2e", submit_host, L)
@@ -643,6 +649,10 @@ def run_ours(args):
                                    "5_synthetic_40x360": "profiles/r02/config5_n*.json (bench.py --config synthetic40x360 --frames 32)"}
             except Exception as e:
                 line["configs"] = {"error": repr(e)}
+        if outputs is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in outputs.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
         print(json.dumps(line))
     for h in lanes:
         h.close()
@@ -697,7 +707,11 @@ def main():
     ap.add_argument("--config", default="seq05", choices=sorted(CONFIGS))
     ap.add_argument("--no-offline-pass", action="store_true", help="skip the informational sequential-pass block")
     ap.add_argument("--no-sweep", action="store_true", help="skip the config-3 preset sweep block")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (map keep mask, per-node counters) "
+                    "as DIR/<name>.npy, to compare two builds on the same seeded inputs")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

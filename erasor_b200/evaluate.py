@@ -3,8 +3,8 @@
 1-NN from every ground-truth point into the estimate, inlier if the distance is below voxelsize*sqrt(3)/2;
 PR = GT-static inliers whose match is static / GT static; RR = (GT dynamic - GT-dynamic inliers whose match is
 dynamic) / GT dynamic; dynamic = SemanticKITTI classes 252..259 carried numerically in `intensity`.
-Host-side quality judge, not part of the path.  tests/test_evaluate.py checks it against the reference's own script
-when /root/reference is present.
+Host-side quality judge, not part of the path.  tests/test_evaluate.py checks it against the stored output of the
+reference's own script (tests/golden/analysis_runner/pr_rr.npz).
 """
 from __future__ import annotations
 

@@ -1,8 +1,7 @@
-"""CPU suite: the PR/RR port (erasor_b200/evaluate.py) against the reference's own scripts/analysis_runner.py
-(run unchanged from /root/reference when it is mounted, i.e. in the build container) on oracle output."""
+"""CPU suite: the PR/RR port (erasor_b200/evaluate.py) against the reference's own scripts/analysis_runner.py, whose
+output on a crop of oracle output is stored in tests/golden/analysis_runner/pr_rr.npz (tests/golden/make_pr_rr_golden.py)."""
 import os
-import subprocess
-import sys
+import re
 
 import numpy as np
 import pytest
@@ -11,7 +10,7 @@ from erasor_b200 import evaluate as E
 from erasor_b200 import params as P
 from erasor_b200 import synth
 
-REF_SCRIPT = "/root/reference/scripts/analysis_runner.py"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "analysis_runner", "pr_rr.npz")
 
 
 @pytest.fixture(scope="module")
@@ -37,18 +36,14 @@ def test_pr_rr_moves_the_right_way(run_pass):
     assert after["RR"] > 30.0 and after["PR"] > 80.0, after      # the pass erases dynamic trails and keeps most static points
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SCRIPT), reason="reference checkout not mounted")
-def test_matches_reference_script(tmp_path, run_pass):
-    gt, est = run_pass
+def test_matches_reference_script(tmp_path):
+    z = np.load(GOLDEN)
     gp, ep_ = str(tmp_path / "gt.pcd"), str(tmp_path / "est.pcd")
-    E.write_pcd_ascii(gp, gt)
-    E.write_pcd_ascii(ep_, est)
-    out = subprocess.run([sys.executable, REF_SCRIPT, "--gt", gp, "--est", ep_], capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
+    E.write_pcd_ascii(gp, z["gt"])
+    E.write_pcd_ascii(ep_, z["est"])
     mine = E.evaluate(E.read_pcd_ascii(gp), E.read_pcd_ascii(ep_))
-    txt = out.stdout
+    txt = str(z["stdout"])
     # the script prints PR / RR / F1 with 3 decimals in a table; find them
-    import re
     nums = [float(x) for x in re.findall(r"-?\d+\.\d+", txt)]
     assert any(abs(v - mine["PR"]) < 2e-3 for v in nums), (mine, txt[-800:])
     assert any(abs(v - mine["RR"]) < 2e-3 for v in nums), (mine, txt[-800:])
