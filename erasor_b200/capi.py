@@ -32,6 +32,7 @@ EXPORTS = [
     "erasor_map_points_device", "erasor_attach_map", "erasor_process_nodes", "erasor_process_nodes_async", "erasor_get_node_stats",
     "erasor_comm_unique_id", "erasor_comm_init", "erasor_comm_destroy", "erasor_allgather_and_keep", "erasor_and_keep_masks",
     "erasor_get_kernel_time_ms", "erasor_reset_kernel_times", "erasor_get_rgpf_profile", "erasor_get_srt_profile",
+    "erasor_process_scans", "erasor_process_scans_async", "erasor_get_scan_queries", "erasor_save_static_map",
     "erasor_updater_create", "erasor_updater_destroy", "erasor_updater_reset", "erasor_updater_last_error", "erasor_updater_process_node", "erasor_updater_prefetch_scan",
     "erasor_updater_map_size", "erasor_updater_get_cloud", "erasor_updater_save_static_map", "erasor_updater_voxelize", "erasor_updater_mapgen_node",
     "erasor_updater_erasor", "erasor_updater_kernel_launch_count", "erasor_updater_get_fused_profile",
@@ -44,6 +45,20 @@ class UpdaterParamsC(ctypes.Structure):
         ("query_voxel_size", c_double), ("map_voxel_size", c_double), ("removal_interval", c_int), ("is_large_scale", c_int),
         ("submap_size", c_double), ("max_range", c_double), ("version", c_int), ("pad_", c_int), ("lidar2body", c_double * 7),
     ]
+
+
+class ScanParamsC(ctypes.Structure):
+    """erasor_scan_params_t"""
+    _fields_ = [("query_voxel_size", c_double), ("lidar2body", c_double * 7)]
+
+
+def scan_params(query_voxel_size: float, lidar2body) -> ScanParamsC:
+    sp = ScanParamsC()
+    sp.query_voxel_size = float(query_voxel_size)
+    l2b = np.asarray(lidar2body, dtype=np.float64).reshape(7)
+    for i in range(7):
+        sp.lidar2body[i] = float(l2b[i])
+    return sp
 
 
 class ErasorError(RuntimeError):
@@ -106,6 +121,11 @@ def _load():
     L.erasor_process_nodes.argtypes = [c_void_p, POINTER(c_double), c_void_p, POINTER(c_uint64), c_int, c_double, c_void_p, c_void_p, c_int]
     L.erasor_process_nodes_async.argtypes = L.erasor_process_nodes.argtypes
     L.erasor_get_node_stats.argtypes = [c_void_p, POINTER(c_uint32), POINTER(c_uint32), POINTER(c_uint32)]
+    L.erasor_process_scans.argtypes = [c_void_p, POINTER(ScanParamsC), POINTER(c_double), c_void_p, POINTER(c_uint64), c_int, c_double, c_void_p,
+                                       c_void_p, c_int]
+    L.erasor_process_scans_async.argtypes = L.erasor_process_scans.argtypes
+    L.erasor_get_scan_queries.argtypes = [c_void_p, c_void_p, c_size_t, POINTER(c_uint64)]
+    L.erasor_save_static_map.argtypes = [c_void_p, c_float, c_void_p, c_size_t, POINTER(c_size_t)]
     L.erasor_comm_unique_id.argtypes = [c_void_p]
     L.erasor_comm_init.argtypes = [c_void_p, c_void_p, c_int, c_int]
     L.erasor_comm_destroy.argtypes = [c_void_p]
@@ -378,6 +398,65 @@ class Handle:
         if rc != OK:
             self._ck(rc)
         self.n_frames = c[5]
+
+    def process_scans(self, poses7, scans, scan_offsets, query_voxel_size: float, lidar2body, voi_max_range: float = 0.0,
+                      want_frame_keep: bool = False, packed_xyz: bool = False):
+        """Node batch on raw LiDAR-frame scans (erasor_process_scans): each scan is voxelised at query_voxel_size and moved to the
+        body frame by lidar2body (x y z qx qy qz qw) on the device, then processed as process_nodes does.  scans: float32 [n,4]
+        (x y z i) or [n,3]; packed_xyz ships them as 12 bytes per point.  Returns (folded keep mask, per-frame masks or None)."""
+        P = np.ascontiguousarray(poses7, dtype=np.float64).reshape(-1, 7)
+        q = np.ascontiguousarray(scans, dtype=np.float32)
+        if q.size == 0:
+            q = q.reshape(0, 4)
+        if q.ndim != 2 or q.shape[1] not in (3, 4):
+            raise ValueError("scans are float32 [n,4] (x y z i) or [n,3] (x y z)")
+        if packed_xyz and q.shape[1] == 4:
+            q = np.ascontiguousarray(q[:, :3])
+        if not packed_xyz and q.shape[1] == 3:
+            raise ValueError("[n,3] scans need packed_xyz=True")
+        so = np.ascontiguousarray(scan_offsets, dtype=np.uint64)
+        F = len(so) - 1
+        assert len(P) == F
+        n = self._map.size
+        keep = np.empty(n, dtype=np.uint8)
+        fk = np.empty((F, n), dtype=np.uint8) if want_frame_keep else None
+        sp = scan_params(query_voxel_size, lidar2body)
+        self._ck(self.L.erasor_process_scans(self.h, ctypes.byref(sp), P.ctypes.data_as(POINTER(c_double)), q.ctypes.data if q.size else None,
+                                             so.ctypes.data_as(POINTER(c_uint64)), F, float(voi_max_range),
+                                             fk.ctypes.data if fk is not None else None, keep.ctypes.data,
+                                             PTR_HOST | (PTR_QUERY_XYZ if packed_xyz else 0)))
+        self.n_frames = F
+        return keep, fk
+
+    def process_scans_ptr(self, sp: ScanParamsC, poses7: np.ndarray, scans_ptr: int, scan_offsets: np.ndarray, voi_max_range: float,
+                          frame_keep_ptr: int, keep_out_ptr: int, ptr_kind: int, asynchronous: bool = False):
+        """Raw-pointer form of process_scans (device tensors or pinned host memory; ptr_kind may carry PTR_QUERY_XYZ).
+        sp: scan_params(...); poses7: contiguous float64 [F,7]; offsets uint64 [F+1]."""
+        assert poses7.dtype == np.float64 and poses7.flags["C_CONTIGUOUS"] and scan_offsets.dtype == np.uint64
+        F = len(scan_offsets) - 1
+        fn = self.L.erasor_process_scans_async if asynchronous else self.L.erasor_process_scans
+        rc = fn(self.h, ctypes.byref(sp), poses7.ctypes.data_as(POINTER(c_double)), scans_ptr or None, scan_offsets.ctypes.data_as(POINTER(c_uint64)),
+                F, float(voi_max_range), frame_keep_ptr or None, keep_out_ptr or None, ptr_kind)
+        if rc != OK:
+            self._ck(rc)
+        self.n_frames = F
+
+    def scan_queries(self):
+        """The voxelised body-frame queries of the last process_scans submission: (x y z float32 [n,3], offsets uint64 [F+1])."""
+        F = self.n_frames
+        off = np.zeros(F + 1, dtype=np.uint64)
+        self._ck(self.L.erasor_get_scan_queries(self.h, None, 0, off.ctypes.data_as(POINTER(c_uint64))))
+        xyz = np.empty((max(int(off[-1]), 1), 3), dtype=np.float32)
+        self._ck(self.L.erasor_get_scan_queries(self.h, xyz.ctypes.data, len(xyz), off.ctypes.data_as(POINTER(c_uint64))))
+        return xyz[:int(off[-1])].copy(), off
+
+    def save_static_map(self, voxel_size: float) -> np.ndarray:
+        """save_static_map of the attached map: voxelize_preserving_labels(map[keep == 1], voxel_size), float32 [n,4]."""
+        n = c_size_t(0)
+        self._ck(self.L.erasor_save_static_map(self.h, float(voxel_size), None, 0, ctypes.byref(n)))
+        out = np.empty((max(n.value, 1), 4), dtype=np.float32)
+        self._ck(self.L.erasor_save_static_map(self.h, float(voxel_size), out.ctypes.data, len(out), ctypes.byref(n)))
+        return out[:n.value].copy()
 
     def node_stats(self):
         F = self.n_frames

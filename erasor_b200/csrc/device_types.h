@@ -27,7 +27,7 @@ struct ChunkDesc {
     uint32_t frame_begin;  // source index of the frame's first point (node mode, map cloud: 0 -- every frame scans the whole map)
     uint32_t bin_begin;    // index of the chunk's first point in the bin-id array (batch mode: == begin; node mode: frame * n_map + begin)
     uint32_t out_base;     // base of the frame's region in the scattered arrays and the per-frame masks (batch: frame_begin; node: frame * n_map)
-    uint32_t pad_;
+    uint32_t pad_;         // (erasor_process_scans, query chunks: the chunk's full length, len being clamped on the device)
 };
 
 // Node mode (map resident in HBM, erasor_process_nodes): what OfflineMapUpdater::fetch_VoI needs per frame

@@ -116,6 +116,10 @@ struct erasor_ctx {
     DevBuf d_poses;                            // node mode: NodePose per frame
     DevBuf d_list_idx, d_list_cnt;             // node mode: per chunk, the map index of every VoI point (dense, map order) and their number
     DevBuf d_pack, d_gather;                   // exchange step: packed keep bits of this rank / of every rank
+    DevBuf d_scan_f4, d_scan_q, d_scan_grid, d_scan_tmp, d_scan_cnt;   // erasor_process_scans: scans widened to float4 (packed x y z input),
+                                                                       // voxelised body-frame queries (at the raw scans' offsets), per-scan
+                                                                       // VoxelGrid state, voxeliser scratch, voxels per scan (+ total)
+    DevBuf d_sv_pts, d_sv_tmp, d_sv_out, d_sv_grid, d_sv_vtmp;        // erasor_save_static_map: kept points, compaction / voxeliser state
     PinnedBuf h_stage, h_pose, h_words;        // h_words: small device -> host read-backs of a submission (pinned: an asynchronous copy into
                                                // pageable memory blocks the launching thread until the whole stream has drained, which
                                                // serialised overlapped handles)
@@ -124,7 +128,7 @@ struct erasor_ctx {
                 &d_zmax, &d_cnt, &d_dst_start, &d_status, &d_action, &d_flag_slot, &d_nflag, &d_recs, &d_nrecs, &d_queue, &d_bucket, &d_frame_rej,
                 &d_map_sorted, &d_map_src, &d_qry_sorted, &d_qry_src, &d_part, &d_scratch, &d_keep, &d_ground, &d_arranged, &d_map_rej, &d_curr_rej,
                 &d_jobs, &d_out_sizes, &d_k5tmp, &d_fence, &d_vox, &d_vox_cnt, &d_vox_start, &d_vox_scratch, &d_frame_rec_base, &d_poses, &d_list_idx, &d_list_cnt, &d_pack,
-                &d_gather};
+                &d_gather, &d_scan_f4, &d_scan_q, &d_scan_grid, &d_scan_tmp, &d_scan_cnt, &d_sv_pts, &d_sv_tmp, &d_sv_out, &d_sv_grid, &d_sv_vtmp};
     }
 
     // batch geometry of the last run
@@ -136,11 +140,12 @@ struct erasor_ctx {
     const float4* cur_qry = nullptr;
     bool     qry_xyz = false;                  // the staged query cloud is packed x y z (ERASOR_PTR_QUERY_XYZ, mask modes)
     std::vector<uint64_t> map_off, qry_off;
-    int      desc_mode = -1;                   // mode the uploaded chunk descriptors were built for (-1: none; 0 cloud, 1 batch masks, 2 node masks)
+    int      desc_mode = -1;                   // mode the uploaded chunk descriptors were built for (-1: none; 0 cloud, 1 batch masks, 2 node masks,
+                                               // 3 node masks on raw scans: query chunks clamped on the device)
     uint64_t desc_epoch = 0;                   // bumped whenever the descriptors are rebuilt (invalidates cached graphs)
     int      stat_F = 0;                       // frames of the last batch call (all its sub-batches): extent of the per-frame counters
     int      f0 = 0;                           // first frame of the sub-batch being submitted
-    struct StepGraph { const void* ptr[8]; size_t fold_n; int kind, mode, f0; uint64_t epoch, alloc; cudaGraphExec_t exec; };
+    struct StepGraph { const void* ptr[8]; size_t fold_n; int kind, mode, f0; uint64_t epoch, alloc; double scan[8]; cudaGraphExec_t exec; };
     std::vector<StepGraph> graphs;             // captured mask-mode steps, one per (pointers, geometry)
     bool     use_graphs = true;
     int      ctas_per_sm = 4;                  // K1 / K2 grid target: one wave of sm_count * ctas_per_sm CTAs (ERASOR_B200_CTAS_PER_SM)
@@ -156,6 +161,7 @@ struct erasor_ctx {
 
     // node mode
     erasor_map_ctx* map = nullptr;
+    int      scan_F = 0;                       // frames of the last submission if it came from erasor_process_scans (0: it did not)
 
     // exchange
     ncclComm_t comm = nullptr;
@@ -274,7 +280,7 @@ int prepare_batch(erasor_ctx* h, const uint64_t* map_off, const uint64_t* qry_of
     h->map_off.assign(map_off, map_off + F + 1);
     h->qry_off.assign(qry_off, qry_off + F + 1);
     const uint32_t CH = choose_chunk(h, map_off, qry_off, F);
-    const bool node = mode == 2;
+    const bool node = mode >= 2;
 
     std::vector<ChunkDesc> chunks;
     std::vector<uint32_t>  range(2 * (size_t)(F + 1)), foff(2 * (size_t)(F + 1));
@@ -289,6 +295,7 @@ int prepare_batch(erasor_ctx* h, const uint64_t* map_off, const uint64_t* qry_of
                 d.len = (uint32_t)std::min<uint64_t>(CH, off[f + 1] - b);
                 d.frame = (uint32_t)f; d.cloud = (uint32_t)c;
                 d.bin_begin = (uint32_t)b; d.out_base = (uint32_t)off[f];
+                d.pad_ = d.len;
                 if (node && c == 0) { d.begin = (uint32_t)(b - off[f]); d.frame_begin = 0u; }      // source = the resident map itself
                 else                { d.begin = (uint32_t)b; d.frame_begin = (uint32_t)off[f]; }
                 chunks.push_back(d);
@@ -860,6 +867,8 @@ struct Submit {
     const NodePose* poses = nullptr;        // mode 2: host array [F]
     uint8_t*        keep_out = nullptr;     // mode 2 (nullable)
     int             f0 = 0;                 // index of the first frame within the caller's batch (per-frame counters)
+    const erasor_scan_params_t* scan = nullptr;   // mode 2 on raw scans (erasor_process_scans): qry_xyzi holds the scans
+    bool            scan_xyz = false;       // ... packed x y z
 };
 
 bool is_pinned_host(const void* p) {
@@ -879,8 +888,20 @@ int submit(erasor_ctx* h, const Submit& S) {
     h->stage = 0;
     h->f0 = S.f0;
     h->qry_xyz = S.qry_xyz;
-    if ((rc = prepare_batch(h, S.map_off, S.qry_off, S.F, S.mode))) return rc;
+    if ((rc = prepare_batch(h, S.map_off, S.qry_off, S.F, S.scan ? 3 : S.mode))) return rc;
     const bool host = S.ptr_kind != ERASOR_PTR_DEVICE;
+    Mat4 T_l2b{};
+    if (S.scan) {
+        Mat4 G{}, I{};                                          // tf_lidar2body_ = geoPose2eigen(pose) * Identity, as the updater builds it
+        pose_to_mat(S.scan->lidar2body, G);
+        for (int i = 0; i < 4; ++i) I.m[5 * i] = 1.0f;
+        mat_mul(G, I, T_l2b);
+        CK(h->d_scan_q.ensure(sizeof(float4) * std::max<size_t>(h->NQ, 1)));
+        CK(h->d_scan_grid.ensure(sizeof(VoxGrid) * (size_t)S.F));
+        CK(h->d_scan_tmp.ensure(voxelize_tmp_bytes((uint32_t)h->NQ, (uint32_t)S.F)));
+        CK(h->d_scan_cnt.ensure(sizeof(uint32_t) * ((size_t)S.F + 1)));
+        if (S.scan_xyz) CK(h->d_scan_f4.ensure(sizeof(float4) * std::max<size_t>(h->NQ, 1)));
+    }
     const size_t n_keep = S.keep_mask ? h->NM : 0;          // bytes of the per-frame mask output
     const size_t n_map_global = S.mode == 2 ? h->map->n : 0;
     if (S.mode == 1 && ((h->NM && !S.map_xyzi) || (h->NQ && !S.qry_xyzi))) { h->err = "null cloud"; return ERASOR_E_INVALID; }
@@ -902,7 +923,29 @@ int submit(erasor_ctx* h, const Submit& S) {
             if ((r = stage_inputs(h, S.map_xyzi, S.qry_xyzi, S.ptr_kind))) return r;
         } else {
             h->cur_map = reinterpret_cast<const float4*>(h->map->d_pts);
-            if ((r = stage_cloud(h, h->d_qry_in, S.qry_xyzi, h->NQ, S.ptr_kind, &h->cur_qry, S.qry_xyz ? 3 * sizeof(float) : sizeof(float4)))) return r;
+            if (!S.scan) {
+                if ((r = stage_cloud(h, h->d_qry_in, S.qry_xyzi, h->NQ, S.ptr_kind, &h->cur_qry, S.qry_xyz ? 3 * sizeof(float) : sizeof(float4)))) return r;
+            } else {
+                // raw scans -> voxelised body-frame queries, all frames in one cooperative launch; frame f's voxels land at its raw
+                // offset, their number in d_scan_cnt[f], and the query chunks (cut from the raw sizes) are clamped to it on the device
+                const float4* raw = nullptr;
+                if ((r = stage_cloud(h, h->d_qry_in, S.qry_xyzi, h->NQ, S.ptr_kind, &raw, S.scan_xyz ? 3 * sizeof(float) : sizeof(float4)))) return r;
+                if (S.scan_xyz) {
+                    h->launches++;
+                    CK(launch_expand_xyz(h->stream, reinterpret_cast<const float*>(raw), h->d_scan_f4.as<float4>(), (uint32_t)h->NQ));
+                    raw = h->d_scan_f4.as<float4>();
+                }
+                FusedJob J{};
+                J.vin = raw; J.vn = (uint32_t)h->NQ; J.leaf = (float)S.scan->query_voxel_size; J.grid = h->d_scan_grid.as<VoxGrid>();
+                J.vtmp = h->d_scan_tmp.p; J.vout = h->d_scan_q.as<float4>(); J.d_n_out = h->d_scan_cnt.as<uint32_t>() + S.F;
+                J.T_out = T_l2b; J.xform_out = 1;
+                J.n_clouds = (uint32_t)S.F; J.cloud_off = h->d_frame_off.as<uint32_t>() + (S.F + 1); J.cloud_nvox = h->d_scan_cnt.as<uint32_t>();
+                J.restore_labels = 0;
+                h->launches += 2;
+                CK(launch_node_fused(h->stream, J, h->sm_count));
+                CK(launch_clamp_query_chunks(h->stream, h->d_chunks.as<ChunkDesc>(), h->n_chunks_map, h->n_chunks_qry, h->d_scan_cnt.as<uint32_t>()));
+                h->cur_qry = h->d_scan_q.as<float4>();
+            }
             CK(cudaMemcpyAsync(h->d_poses.p, h->h_pose.p, sizeof(NodePose) * (size_t)S.F, cudaMemcpyHostToDevice, h->stream));
         }
         uint8_t* d_keep = nullptr;
@@ -936,10 +979,12 @@ int submit(erasor_ctx* h, const Submit& S) {
         erasor_ctx::StepGraph key{};
         key.ptr[0] = S.map_xyzi; key.ptr[1] = S.qry_xyzi; key.ptr[2] = S.keep_mask; key.ptr[3] = S.fold_index; key.ptr[4] = S.fold_global;
         key.ptr[5] = S.keep_out; key.ptr[6] = S.mode == 2 ? (const void*)h->map : nullptr; key.ptr[7] = with_c ? (const void*)h : nullptr;
-        key.fold_n = S.fold_n; key.kind = S.ptr_kind | (S.qry_xyz ? ERASOR_PTR_QUERY_XYZ : 0); key.mode = S.mode; key.f0 = S.f0; key.epoch = h->desc_epoch; key.alloc = h->alloc_epoch;
+        key.fold_n = S.fold_n; key.kind = S.ptr_kind | (S.qry_xyz || S.scan_xyz ? ERASOR_PTR_QUERY_XYZ : 0); key.mode = S.scan ? 3 : S.mode; key.f0 = S.f0;
+        key.epoch = h->desc_epoch; key.alloc = h->alloc_epoch;
+        for (int i = 0; i < 8; ++i) key.scan[i] = S.scan ? (i == 0 ? S.scan->query_voxel_size : S.scan->lidar2body[i - 1]) : 0.0;   // baked into the voxeliser's launch
         auto same = [&](const erasor_ctx::StepGraph& g) {
             return std::equal(g.ptr, g.ptr + 8, key.ptr) && g.fold_n == key.fold_n && g.kind == key.kind && g.mode == key.mode && g.f0 == key.f0 &&
-                   g.epoch == key.epoch && g.alloc == key.alloc;
+                   g.epoch == key.epoch && g.alloc == key.alloc && std::equal(g.scan, g.scan + 8, key.scan);
         };
         cudaGraphExec_t exec = nullptr;
         for (auto& g : h->graphs) if (same(g)) exec = g.exec;
@@ -986,6 +1031,7 @@ int submit(erasor_ctx* h, const Submit& S) {
         else if (S.fold_global) h->last.fold = K4Fold{S.fold_global, S.fold_index, (uint32_t)std::min<size_t>(S.fold_n, 0xFFFFFFFFu), 0u};
         else                    h->last.fold = K4Fold{nullptr, nullptr, 0u, 0u};
     }
+    h->scan_F = S.scan ? S.F : 0;
     h->pending = true;
     return ERASOR_OK;
 }
@@ -1035,8 +1081,10 @@ int process_frames_impl(erasor_handle_t h, const float* map_xyzi, const uint64_t
     return async ? ERASOR_OK : erasor_wait(h);
 }
 
+// scan: erasor_process_scans -- query_xyzi holds raw scans, voxelised and moved to the body frame on the device first
 int process_nodes_impl(erasor_handle_t h, const double* poses7, const float* query_xyzi, const uint64_t* query_offsets, int n_frames,
-                       double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind, bool async) {
+                       double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind, bool async,
+                       const erasor_scan_params_t* scan = nullptr) {
     if (!h || !poses7 || !query_offsets) { if (h) h->err = "null argument"; return ERASOR_E_INVALID; }
     if (!h->map) { h->err = "erasor_process_nodes: no map attached (erasor_attach_map)"; return ERASOR_E_STATE; }
     if (n_frames <= 0) { h->err = "n_frames must be positive"; return ERASOR_E_INVALID; }
@@ -1069,7 +1117,8 @@ int process_nodes_impl(erasor_handle_t h, const double* poses7, const float* que
         poses.resize(F);
         for (int f = 0; f < F; ++f) node_pose_of(poses7 + 7 * (size_t)(f0 + f), range, poses[f]);
         Submit S;
-        S.mode = 2; S.F = F; S.ptr_kind = ptr_kind; S.f0 = f0; S.qry_xyz = qxyz;
+        S.mode = 2; S.F = F; S.ptr_kind = ptr_kind; S.f0 = f0; S.qry_xyz = scan ? false : qxyz;
+        S.scan = scan; S.scan_xyz = scan ? qxyz : false;
         S.map_off = mo.data(); S.qry_off = qo.data();
         S.qry_xyzi = query_xyzi ? query_xyzi + (qxyz ? 3 : 4) * q0 : nullptr;
         S.keep_mask = frame_keep ? frame_keep + (size_t)f0 * N : nullptr;
@@ -1225,9 +1274,98 @@ int erasor_process_nodes_async(erasor_handle_t h, const double* poses7, const fl
     return process_nodes_impl(h, poses7, query_xyzi, query_offsets, n_frames, voi_max_range, frame_keep, keep_out, ptr_kind, true);
 }
 
+namespace {
+int process_scans_impl(erasor_handle_t h, const erasor_scan_params_t* sp, const double* poses7, const float* scans, const uint64_t* scan_offsets,
+                       int n_frames, double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind, bool async) {
+    if (!h) return ERASOR_E_INVALID;
+    if (!sp || !poses7 || !scan_offsets) { h->err = "null argument"; return ERASOR_E_INVALID; }
+    const double leaf = sp->query_voxel_size;
+    if (!(leaf > 0.0) || !std::isfinite(leaf) || !((float)leaf > 0.0f) || !std::isfinite((float)leaf)) { h->err = "query_voxel_size must be positive and finite"; return ERASOR_E_INVALID; }
+    double qn = 0.0;
+    for (int i = 0; i < 7; ++i) { if (!std::isfinite(sp->lidar2body[i])) { h->err = "lidar2body must be finite"; return ERASOR_E_INVALID; } }
+    for (int i = 3; i < 7; ++i) qn += sp->lidar2body[i] * sp->lidar2body[i];
+    if (!(qn > 0.0)) { h->err = "lidar2body: zero quaternion"; return ERASOR_E_INVALID; }
+    if (n_frames > 0) {
+        for (size_t i = 0; i < 7 * (size_t)n_frames; ++i) if (!std::isfinite(poses7[i])) { h->err = "poses must be finite"; return ERASOR_E_INVALID; }
+        for (int f = 0; f < n_frames; ++f) if (scan_offsets[f + 1] < scan_offsets[f]) { h->err = "offsets must be non-decreasing"; return ERASOR_E_INVALID; }
+        if (scan_offsets[n_frames] > scan_offsets[0] && !scans) { h->err = "null cloud"; return ERASOR_E_INVALID; }
+    }
+    return process_nodes_impl(h, poses7, scans, scan_offsets, n_frames, voi_max_range, frame_keep, keep_out, ptr_kind, async, sp);
+}
+}  // namespace
+
+int erasor_process_scans(erasor_handle_t h, const erasor_scan_params_t* sp, const double* poses7, const float* scans, const uint64_t* scan_offsets,
+                         int n_frames, double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind) {
+    return process_scans_impl(h, sp, poses7, scans, scan_offsets, n_frames, voi_max_range, frame_keep, keep_out, ptr_kind, false);
+}
+int erasor_process_scans_async(erasor_handle_t h, const erasor_scan_params_t* sp, const double* poses7, const float* scans, const uint64_t* scan_offsets,
+                               int n_frames, double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind) {
+    return process_scans_impl(h, sp, poses7, scans, scan_offsets, n_frames, voi_max_range, frame_keep, keep_out, ptr_kind, true);
+}
+
+int erasor_get_scan_queries(erasor_handle_t h, float* xyz, size_t cap, uint64_t* offsets) {
+    if (!h) return ERASOR_E_INVALID;
+    if (!offsets) { h->err = "null argument"; return ERASOR_E_INVALID; }
+    if (h->scan_F <= 0) { h->err = "the last submission did not come from erasor_process_scans"; return ERASOR_E_STATE; }
+    int rc;
+    if ((rc = erasor_wait(h))) return rc;
+    const int F = h->scan_F;
+    std::vector<uint32_t> cnt((size_t)F);
+    CK(cudaMemcpy(cnt.data(), h->d_scan_cnt.p, sizeof(uint32_t) * (size_t)F, cudaMemcpyDeviceToHost));
+    offsets[0] = 0;
+    for (int f = 0; f < F; ++f) offsets[f + 1] = offsets[f] + cnt[f];
+    if (!xyz) return ERASOR_OK;
+    if (cap < offsets[F]) { h->err = "output buffer too small"; return ERASOR_E_CAPACITY; }
+    std::vector<float4> tmp;
+    for (int f = 0; f < F; ++f) {
+        tmp.resize(cnt[f]);
+        if (cnt[f]) CK(cudaMemcpy(tmp.data(), h->d_scan_q.as<float4>() + h->qry_off[f], sizeof(float4) * cnt[f], cudaMemcpyDeviceToHost));
+        float* o = xyz + 3 * offsets[f];
+        for (uint32_t i = 0; i < cnt[f]; ++i) { o[3 * i] = tmp[i].x; o[3 * i + 1] = tmp[i].y; o[3 * i + 2] = tmp[i].z; }
+    }
+    return ERASOR_OK;
+}
+
+// OfflineMapUpdater::save_static_map (OfflineMapUpdater.cpp:174-196) on the attached map: keep-byte compaction, then U3 with labels
+int erasor_save_static_map(erasor_handle_t h, float voxel_size, float* out_xyzi, size_t cap, size_t* n) {
+    if (!h) return ERASOR_E_INVALID;
+    if (!n) { h->err = "null argument"; return ERASOR_E_INVALID; }
+    if (!h->map) { h->err = "erasor_save_static_map: no map attached (erasor_attach_map)"; return ERASOR_E_STATE; }
+    if (!(voxel_size > 0.0f) || !std::isfinite(voxel_size)) { h->err = "voxel_size must be positive and finite"; return ERASOR_E_INVALID; }
+    int rc;
+    if ((rc = erasor_wait(h))) return rc;
+    CK(cudaStreamSynchronize(h->map->st));
+    const size_t N = h->map->n;
+    CK(h->d_sv_pts.ensure(sizeof(float4) * std::max<size_t>(N, 1)));
+    CK(h->d_sv_tmp.ensure(sizeof(uint32_t) * (partition_tmp_words((uint32_t)N) + 2)));
+    uint32_t* d_cnt = h->d_sv_tmp.as<uint32_t>();                   // [0] kept points, [1] voxels, [2..) chunk counters
+    h->launches += 3;
+    CK(launch_compact_keep(h->stream, h->map->d_pts, h->map->d_keep, (uint32_t)N, h->d_sv_pts.as<float4>(), d_cnt, d_cnt + 2));
+    uint32_t* w = h->h_words.as<uint32_t>();
+    CK(cudaMemcpyAsync(w + 12, d_cnt, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const uint32_t nk = w[12];
+    CK(h->d_sv_out.ensure(sizeof(float4) * std::max<size_t>(nk, 1)));
+    CK(h->d_sv_grid.ensure(sizeof(VoxGrid)));
+    CK(h->d_sv_vtmp.ensure(voxelize_tmp_bytes(nk)));
+    FusedJob J{};
+    J.vin = h->d_sv_pts.as<float4>(); J.vn = nk; J.leaf = voxel_size; J.grid = h->d_sv_grid.as<VoxGrid>(); J.vtmp = h->d_sv_vtmp.p;
+    J.vout = h->d_sv_out.as<float4>(); J.d_n_out = d_cnt + 1; J.xform_out = 0;
+    h->launches++;
+    CK(launch_node_fused(h->stream, J, h->sm_count));
+    CK(cudaMemcpyAsync(w + 13, d_cnt + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const uint32_t nv = w[13];
+    *n = nv;
+    if (!out_xyzi) return ERASOR_OK;
+    if (cap < nv) { h->err = "output buffer too small"; return ERASOR_E_CAPACITY; }
+    if (nv) CK(cudaMemcpy(out_xyzi, h->d_sv_out.p, sizeof(float4) * nv, cudaMemcpyDeviceToHost));
+    return ERASOR_OK;
+}
+
 int erasor_get_node_stats(erasor_handle_t h, uint32_t* n_voi_points, uint32_t* n_flagged_bins, uint32_t* n_rejected_points) {
     if (!h) return ERASOR_E_INVALID;
-    if (h->F <= 0 || h->desc_mode != 2) { h->err = "no node batch has run"; return ERASOR_E_STATE; }
+    if (h->F <= 0 || h->desc_mode < 2) { h->err = "no node batch has run"; return ERASOR_E_STATE; }
     int rc;
     if ((rc = erasor_wait(h))) return rc;
     if (n_voi_points) {

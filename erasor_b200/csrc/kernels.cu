@@ -2388,4 +2388,19 @@ cudaError_t launch_fill_u8(cudaStream_t st, uint8_t* p, size_t n, uint8_t v) {
     return cudaGetLastError();
 }
 
+// erasor_process_scans: the query chunks were cut on the host from the raw scan sizes (an upper bound of the voxel counts);
+// set every query chunk's length from its full length (pad_) and the frame's voxel count written by the batched voxeliser
+__global__ void __launch_bounds__(256) k_clamp_query_chunks(ChunkDesc* __restrict__ chunks, uint32_t first, uint32_t n, const uint32_t* __restrict__ count) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    ChunkDesc& d = chunks[first + i];
+    const uint32_t c = count[d.frame], s = d.begin - d.frame_begin;
+    d.len = c > s ? min(d.pad_, c - s) : 0u;
+}
+cudaError_t launch_clamp_query_chunks(cudaStream_t st, ChunkDesc* chunks, uint32_t first, uint32_t n, const uint32_t* count) {
+    if (n == 0) return cudaSuccess;
+    k_clamp_query_chunks<<<(n + 255) / 256, 256, 0, st>>>(chunks, first, n, count);
+    return cudaGetLastError();
+}
+
 }  // namespace erasor

@@ -75,6 +75,8 @@ cudaError_t launch_k5(cudaStream_t st, int B, int version, int skip_voxelize, co
 
 cudaError_t launch_fold_keep(cudaStream_t st, const uint8_t* keep, const uint32_t* voi_index, size_t n, uint8_t* global_keep, size_t n_global);
 cudaError_t launch_fill_u8(cudaStream_t st, uint8_t* p, size_t n, uint8_t v);
+// chunks[first .. first + n): len = min(full length in pad_, what is left of count[frame] from the chunk's start)
+cudaError_t launch_clamp_query_chunks(cudaStream_t st, ChunkDesc* chunks, uint32_t first, uint32_t n, const uint32_t* count);
 // exchange step of the frame-sharded job: pack the keep bytes into bits, AND the all-gathered words of every rank, unpack
 cudaError_t launch_pack_keep_bits(cudaStream_t st, const uint8_t* keep, size_t n, uint32_t* words);
 cudaError_t launch_and_unpack_keep(cudaStream_t st, const uint32_t* gathered, int n_ranks, size_t n, uint8_t* keep);

@@ -250,11 +250,91 @@ __device__ __forceinline__ uint32_t cta_sum(uint32_t c, uint32_t* s_w /*[FW]*/) 
     return t;
 }
 
+// batched U3: the cloud that point (or sorted position) e belongs to = the first f with off[f + 1] > e (empty clouds are skipped)
+__device__ __forceinline__ uint32_t cloud_of(const uint32_t* __restrict__ off, uint32_t F, uint32_t e) {
+    uint32_t lo = 0, hi = F;
+    while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (off[mid + 1] <= e) lo = mid + 1; else hi = mid; }
+    return lo;
+}
+// first index in a[0..n) with a[i] >= x (a ascending)
+__device__ __forceinline__ uint32_t lower_bound_u32(const uint32_t* __restrict__ a, uint32_t n, uint32_t x) {
+    uint32_t lo = 0, hi = n;
+    while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (a[mid] < x) lo = mid + 1; else hi = mid; }
+    return lo;
+}
+
+// getMinMax3D of in[b0..b1) by the whole grid: this CTA's partial (order-preserving encodings, min x y z then max x y z) to out6
+__device__ __forceinline__ void cta_minmax(const float4* __restrict__ in, uint32_t b0, uint32_t b1, uint32_t* s_c, uint32_t* out6) {
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    uint32_t mn[3] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu}, mx[3] = {0u, 0u, 0u};
+    for (uint32_t i = b0 + blockIdx.x * FT + tid; i < b1; i += gridDim.x * FT) {
+        const float4 p = in[i];
+        const uint32_t a = f2ord(p.x + 0.0f), b = f2ord(p.y + 0.0f), c = f2ord(p.z + 0.0f);
+        mn[0] = min(mn[0], a); mx[0] = max(mx[0], a);
+        mn[1] = min(mn[1], b); mx[1] = max(mx[1], b);
+        mn[2] = min(mn[2], c); mx[2] = max(mx[2], c);
+    }
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const uint32_t a = __reduce_min_sync(FULL_MASK, mn[k]), b = __reduce_max_sync(FULL_MASK, mx[k]);
+        if (lane == 0) { s_c[warp * 6 + k] = a; s_c[warp * 6 + 3 + k] = b; }
+    }
+    __syncthreads();
+    if (tid < 6) {
+        uint32_t r = (tid < 3) ? 0xFFFFFFFFu : 0u;
+        for (int w = 0; w < FW; ++w) r = (tid < 3) ? min(r, s_c[w * 6 + tid]) : max(r, s_c[w * 6 + tid]);
+        out6[tid] = r;
+    }
+    __syncthreads();
+}
+
+// pcl::VoxelGrid set-up of one cloud of n points from its min / max (s_w[0..6), order-preserving encodings); one thread
+__device__ void vox_grid_setup(VoxGrid* g, float leaf, uint32_t n, const uint32_t* s_w) {
+    g->n_vox = 0; g->overflow = 0; g->npass = 0;
+    const float inv = FD(1.0f, leaf);
+    g->leaf = leaf; g->inv = inv;
+    if (n == 0) {
+        for (int k = 0; k < 3; ++k) { g->mn[k] = 0xFFFFFFFFu; g->mx[k] = 0u; g->div[k] = 1; g->min_b[k] = 0; }
+        return;
+    }
+    float mnf[3], mxf[3];
+    for (int k = 0; k < 3; ++k) {
+        g->mn[k] = s_w[k]; g->mx[k] = s_w[3 + k];
+        mnf[k] = ord2f(s_w[k]); mxf[k] = ord2f(s_w[3 + k]);
+    }
+    const long long dx = (long long)FM(FS(mxf[0], mnf[0]), inv) + 1;
+    const long long dy = (long long)FM(FS(mxf[1], mnf[1]), inv) + 1;
+    const long long dz = (long long)FM(FS(mxf[2], mnf[2]), inv) + 1;
+    const int ovf = (dx * dy * dz) > 2147483647LL ? 1 : 0;
+    g->overflow = ovf;
+    unsigned long long cells = 1ull;
+    for (int k = 0; k < 3; ++k) {
+        g->min_b[k] = (int)floorf(FM(mnf[k], inv));
+        const int max_b = (int)floorf(FM(mxf[k], inv));
+        g->div[k] = max_b - g->min_b[k] + 1;
+        cells *= (unsigned long long)(unsigned)g->div[k];
+    }
+    // radix passes the keys need: keys are < cells (int32 arithmetic as in PCL), or < n in the overflow case
+    unsigned long long lim = ovf ? (unsigned long long)n : cells;
+    int bits = 32;
+    if (lim <= 0x80000000ull) { bits = 1; while ((1ull << bits) < lim) ++bits; }
+    g->npass = (bits + RB - 1) / RB;
+}
+
+// pcl::VoxelGrid key of point p (local: its index within its cloud, the key of the overflow case)
+__device__ __forceinline__ uint32_t vox_key(int ovf, float inv, float mb0, float mb1, float mb2, int d0, int d01, float4 p, uint32_t local) {
+    if (ovf) return local;      // "Leaf size is too small": output = input, one point per voxel in cloud order
+    const int ijk0 = (int)FS(floorf(FM(p.x, inv)), mb0);
+    const int ijk1 = (int)FS(floorf(FM(p.y, inv)), mb1);
+    const int ijk2 = (int)FS(floorf(FM(p.z, inv)), mb2);
+    return (uint32_t)(ijk0 + ijk1 * d0 + ijk2 * d01);
+}
+
 struct VoxPlan {                          // carve-up of the voxeliser's scratch (host and device agree through this one function)
-    uint32_t *key_a, *idx_a, *key_b, *idx_b, *cnt_x, *cnt_y, *tot, *chunk, *vstart, *vkey, *partial;
+    uint32_t *key_a, *idx_a, *key_b, *idx_b, *cnt_x, *cnt_y, *tot, *chunk, *vstart, *vkey, *partial, *cvox;
     uint32_t seg, nseg;
 };
-__host__ __device__ inline VoxPlan vox_plan(void* tmp, uint32_t n) {
+__host__ __device__ inline VoxPlan vox_plan(void* tmp, uint32_t n, uint32_t n_clouds = 1) {
     VoxPlan p;
     uint32_t* w = reinterpret_cast<uint32_t*>(tmp);
     p.seg  = rs_seg_len(n);
@@ -267,10 +347,16 @@ __host__ __device__ inline VoxPlan vox_plan(void* tmp, uint32_t n) {
     p.chunk = p.tot + RD;                                            // (n + PART_CHUNK - 1) / PART_CHUNK + 1
     p.vstart = p.chunk + ((size_t)(n + PART_CHUNK - 1) / PART_CHUNK + 1);   // n + 2
     p.vkey   = p.vstart + ((size_t)n + 2);                            // n + 2
-    p.partial = p.vkey + ((size_t)n + 2);                             // 6 * kFusedMaxGrid
+    p.partial = p.vkey + ((size_t)n + 2);                             // 6 * kFusedMaxGrid per cloud
+    p.cvox    = p.partial + (size_t)6 * kFusedMaxGrid * n_clouds;     // batched: first voxel of every non-empty cloud
     return p;
 }
 
+// BATCH = false: one cloud (FusedJob.vin[0..vn)) plus the optional U1 partition -- the sequential updater's form.
+// BATCH = true:  FusedJob.n_clouds clouds in one launch.  The phases are the same; per cloud they keep their own min / max,
+// grid and key, and after the key passes the stable radix sort runs the cloud id as its most significant digit(s), so
+// every cloud's points end up contiguous, in ascending key, members in cloud order -- what one call per cloud gives.
+template <bool BATCH>
 __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
     cg::grid_group grid = cg::this_grid();
     extern __shared__ uint32_t s_c[];        // [FW][RD] next free destination per digit, one row per warp (also the min/max staging)
@@ -279,7 +365,10 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const uint32_t G = gridDim.x, bid = blockIdx.x;
     const uint32_t n = J.vn, pn = J.pn;
-    const VoxPlan vp = vox_plan(J.vtmp, n);
+    const uint32_t NC = BATCH ? J.n_clouds : 1u;
+    const uint32_t* __restrict__ coff = J.cloud_off;
+    const bool has_part = !BATCH && J.has_part;
+    const VoxPlan vp = vox_plan(J.vtmp, n, NC);
     const uint32_t nseg = vp.nseg, SEG = vp.seg;
     VoxGrid* g = J.grid;
     const uint32_t pchunks = (pn + PART_CHUNK - 1) / PART_CHUNK;
@@ -290,28 +379,19 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
     // ---- phase 0: getMinMax3D partials per CTA | partition: selected points per chunk ----
     if (n) {
         for (uint32_t i = bid * FT + tid; i < 2u * RD * (nseg + 1u); i += G * FT) vp.cnt_x[i] = 0u;      // both histogram matrices (contiguous)
-        uint32_t mn[3] = {0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu}, mx[3] = {0u, 0u, 0u};
-        for (uint32_t i = bid * FT + tid; i < n; i += G * FT) {
-            const float4 p = J.vin[i];
-            const uint32_t a = f2ord(p.x + 0.0f), b = f2ord(p.y + 0.0f), c = f2ord(p.z + 0.0f);
-            mn[0] = min(mn[0], a); mx[0] = max(mx[0], a);
-            mn[1] = min(mn[1], b); mx[1] = max(mx[1], b);
-            mn[2] = min(mn[2], c); mx[2] = max(mx[2], c);
+        if (!BATCH) {
+            cta_minmax(J.vin, 0u, n, s_c, vp.partial + bid * 6);
+        } else {
+            for (uint32_t f = 0; f < NC; ++f) {                                                  // per cloud: partial [f][bid][6]
+                const uint32_t o0 = coff[f], o1 = coff[f + 1];
+                if (o0 < o1) cta_minmax(J.vin, o0, o1, s_c, vp.partial + ((size_t)f * G + bid) * 6);
+            }
         }
-#pragma unroll
-        for (int k = 0; k < 3; ++k) {
-            const uint32_t a = __reduce_min_sync(FULL_MASK, mn[k]), b = __reduce_max_sync(FULL_MASK, mx[k]);
-            if (lane == 0) { s_c[warp * 6 + k] = a; s_c[warp * 6 + 3 + k] = b; }
-        }
-        __syncthreads();
-        if (tid < 6) {
-            uint32_t r = (tid < 3) ? 0xFFFFFFFFu : 0u;
-            for (int w = 0; w < FW; ++w) r = (tid < 3) ? min(r, s_c[w * 6 + tid]) : max(r, s_c[w * 6 + tid]);
-            vp.partial[bid * 6 + tid] = r;
-        }
-        __syncthreads();
     }
-    if (J.has_part) {
+    if (BATCH) {
+        for (uint32_t f = bid * FT + tid; f < NC; f += G * FT) J.cloud_nvox[f] = 0u;
+    }
+    if (has_part) {
         for (uint32_t vb = bid; vb < pchunks; vb += G) {
             const uint32_t b0 = vb * PART_CHUNK, b1 = min(pn, b0 + PART_CHUNK);
             uint32_t c = 0;
@@ -324,76 +404,60 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
     PH(1);
 
     // ---- phase 1: VoxelGrid set-up (CTA 0) | partition: chunk offsets (last CTA) ----
-    if (bid == 0) {
-        if (n && warp < 6) {                    // reduce the per-CTA partials: warp k < 3 the minimum of axis k, warps 3..5 the maxima
+    for (uint32_t f = bid; f < NC; f += G) {      // (one cloud: CTA 0)
+        const uint32_t nf = BATCH ? coff[f + 1] - coff[f] : n;
+        if (nf && warp < 6) {                   // reduce the per-CTA partials: warp k < 3 the minimum of axis k, warps 3..5 the maxima
+            const uint32_t* part = vp.partial + (size_t)f * G * 6;
             uint32_t r = (warp < 3) ? 0xFFFFFFFFu : 0u;
-            for (uint32_t c = lane; c < G; c += 32) r = (warp < 3) ? min(r, vp.partial[c * 6 + warp]) : max(r, vp.partial[c * 6 + warp]);
+            for (uint32_t c = lane; c < G; c += 32) r = (warp < 3) ? min(r, part[c * 6 + warp]) : max(r, part[c * 6 + warp]);
             r = (warp < 3) ? __reduce_min_sync(FULL_MASK, r) : __reduce_max_sync(FULL_MASK, r);
             if (lane == 0) s_w[warp] = r;
         }
         __syncthreads();
         if (tid == 0) {
-            g->n_vox = 0; g->overflow = 0; g->npass = 0;
-            const float inv = FD(1.0f, J.leaf);
-            g->leaf = J.leaf; g->inv = inv;
-            if (n == 0) {
-                for (int k = 0; k < 3; ++k) { g->mn[k] = 0xFFFFFFFFu; g->mx[k] = 0u; g->div[k] = 1; g->min_b[k] = 0; }
-                *J.d_n_out = 0u;
-            } else {
-                float mnf[3], mxf[3];
-                for (int k = 0; k < 3; ++k) {
-                    g->mn[k] = s_w[k]; g->mx[k] = s_w[3 + k];
-                    mnf[k] = ord2f(s_w[k]); mxf[k] = ord2f(s_w[3 + k]);
-                }
-                const long long dx = (long long)FM(FS(mxf[0], mnf[0]), inv) + 1;
-                const long long dy = (long long)FM(FS(mxf[1], mnf[1]), inv) + 1;
-                const long long dz = (long long)FM(FS(mxf[2], mnf[2]), inv) + 1;
-                const int ovf = (dx * dy * dz) > 2147483647LL ? 1 : 0;
-                g->overflow = ovf;
-                unsigned long long cells = 1ull;
-                for (int k = 0; k < 3; ++k) {
-                    g->min_b[k] = (int)floorf(FM(mnf[k], inv));
-                    const int max_b = (int)floorf(FM(mxf[k], inv));
-                    g->div[k] = max_b - g->min_b[k] + 1;
-                    cells *= (unsigned long long)(unsigned)g->div[k];
-                }
-                // radix passes the keys need: keys are < cells (int32 arithmetic as in PCL), or < n in the overflow case
-                unsigned long long lim = ovf ? (unsigned long long)n : cells;
-                int bits = 32;
-                if (lim <= 0x80000000ull) { bits = 1; while ((1ull << bits) < lim) ++bits; }
-                g->npass = (bits + RB - 1) / RB;
-            }
+            vox_grid_setup(g + f, J.leaf, nf, s_w);
+            if (n == 0 && f == 0) *J.d_n_out = 0u;
         }
         __syncthreads();
     }
-    if (J.has_part && bid == G - 1) cta_scan_u32(J.chunk_tmp, pchunks, J.d_total_sel, s_part);
+    if (has_part && bid == G - 1) cta_scan_u32(J.chunk_tmp, pchunks, J.d_total_sel, s_part);
     grid.sync();
     PH(2);
 
     // ---- phase 2: voxel keys + digit-0 histogram, one warp per 1024-point segment | partition: stable scatter ----
-    const int npass = n ? g->npass : 0;
+    // batched: the key passes every cloud needs, then the cloud id's digits
+    int npk = 0, npass = 0;
+    if (!BATCH) {
+        npass = n ? g->npass : 0;
+        npk = npass;
+    } else if (n) {
+        for (uint32_t f = lane; f < NC; f += 32) npk = max(npk, g[f].npass);
+        npk = __reduce_max_sync(FULL_MASK, npk);
+        const int cbits = NC > 1 ? 32 - __clz(NC - 1) : 0;
+        npass = npk + (cbits + RB - 1) / RB;
+    }
     uint32_t* const my_c = s_c + warp * RD;
-    if (n) {
+    if (n && !BATCH) {
         const int ovf = g->overflow;
         const float inv = g->inv;
         const float mb0 = (float)g->min_b[0], mb1 = (float)g->min_b[1], mb2 = (float)g->min_b[2];
         const int d0 = g->div[0], d01 = g->div[0] * g->div[1];
         for (uint32_t e = bid * FT + tid; e < n; e += G * FT) {
-            const float4 p = J.vin[e];
-            uint32_t k;
-            if (ovf) {
-                k = e;      // "Leaf size is too small": output = input, one point per voxel in cloud order
-            } else {
-                const int ijk0 = (int)FS(floorf(FM(p.x, inv)), mb0);
-                const int ijk1 = (int)FS(floorf(FM(p.y, inv)), mb1);
-                const int ijk2 = (int)FS(floorf(FM(p.z, inv)), mb2);
-                k = (uint32_t)(ijk0 + ijk1 * d0 + ijk2 * d01);
-            }
+            const uint32_t k = vox_key(ovf, inv, mb0, mb1, mb2, d0, d01, J.vin[e], e);
             vp.key_a[e] = k; vp.idx_a[e] = e;
             atomicAdd(&vp.cnt_x[(size_t)(k & (RD - 1u)) * nseg + e / SEG], 1u);      // pass 0's histogram (counts: order-free)
         }
+    } else if (n) {
+        for (uint32_t e = bid * FT + tid; e < n; e += G * FT) {
+            const uint32_t f = cloud_of(coff, NC, e);
+            const VoxGrid* gf = g + f;
+            const uint32_t k = vox_key(gf->overflow, gf->inv, (float)gf->min_b[0], (float)gf->min_b[1], (float)gf->min_b[2], gf->div[0],
+                                       gf->div[0] * gf->div[1], J.vin[e], e - coff[f]);
+            vp.key_a[e] = k; vp.idx_a[e] = e;
+            atomicAdd(&vp.cnt_x[(size_t)(k & (RD - 1u)) * nseg + e / SEG], 1u);
+        }
     }
-    if (J.has_part) {
+    if (has_part) {
         for (uint32_t vb = bid; vb < pchunks; vb += G) {
             const uint32_t b0 = vb * PART_CHUNK, b1 = min(pn, b0 + PART_CHUNK);
             uint32_t sel_base = J.chunk_tmp[vb];
@@ -486,7 +550,8 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
                     unsigned my_peers = 0u;
                     uint32_t dst_o = 0u;
                     if (valid) {
-                        const uint32_t d = (kk[r] >> shift) & (RD - 1u);
+                        const uint32_t d = (!BATCH || pass < npk) ? (kk[r] >> shift) & (RD - 1u)
+                                                                  : (cloud_of(coff, NC, vv[r]) >> ((pass - npk) * RB)) & (RD - 1u);
                         const unsigned peers = __match_any_sync(vm, d);
                         const uint32_t base = my_c[d];
                         __syncwarp(vm);
@@ -498,7 +563,10 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
                     if (more) {
                         // next pass's histogram: one RED per run of equal digits when the whole run lands in one counter (the usual
                         // case -- neighbouring voxels share their upper key bits), else one per point
-                        const uint32_t slot = valid ? ((kk[r] >> (shift + RB)) & (RD - 1u)) * nseg + dst_o / SEG : 0xFFFFFFFFu;
+                        uint32_t nd = 0u;
+                        if (valid) nd = (!BATCH || pass + 1 < npk) ? (kk[r] >> (shift + RB)) & (RD - 1u)
+                                                                   : (cloud_of(coff, NC, vv[r]) >> ((pass + 1 - npk) * RB)) & (RD - 1u);
+                        const uint32_t slot = valid ? nd * nseg + dst_o / SEG : 0xFFFFFFFFu;
                         const int      lead = valid ? __ffs(my_peers) - 1 : lane;
                         const uint32_t lslot = __shfl_sync(FULL_MASK, slot, lead);
                         const unsigned differ = __ballot_sync(FULL_MASK, valid && slot != lslot);
@@ -525,7 +593,8 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
     for (uint32_t vb = bid; vb < hchunks; vb += G) {
         const uint32_t b0 = vb * PART_CHUNK, b1 = min(n, b0 + PART_CHUNK);
         uint32_t c = 0;
-        for (uint32_t i = b0 + tid; i < b1; i += FT) c += (i == 0 || skey[i] != skey[i - 1]) ? 1u : 0u;
+        for (uint32_t i = b0 + tid; i < b1; i += FT)
+            c += (i == 0 || skey[i] != skey[i - 1] || (BATCH && cloud_of(coff, NC, i) != cloud_of(coff, NC, i - 1))) ? 1u : 0u;
         const uint32_t t = cta_sum(c, s_w);
         if (tid == 0) vp.chunk[vb] = t;
     }
@@ -534,16 +603,20 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
     grid.sync();
     PH(13);
     const uint32_t n_vox = *J.d_n_out;
-    if (bid == 0 && tid == 0) { g->n_vox = n_vox; vp.vstart[n_vox] = n; }
+    if (bid == 0 && tid == 0) { if (!BATCH) g->n_vox = n_vox; vp.vstart[n_vox] = n; }
     for (uint32_t vb = bid; vb < hchunks; vb += G) {
         const uint32_t b0 = vb * PART_CHUNK, b1 = min(n, b0 + PART_CHUNK);
         uint32_t base = vp.chunk[vb];
         for (uint32_t r0 = b0; r0 < b1; r0 += FT) {
             const uint32_t i = r0 + tid;
-            const bool hd = (i < b1) && (i == 0 || skey[i] != skey[i - 1]);
+            // (batched: the sort left cloud f at positions [cloud_off[f], cloud_off[f + 1]), so a cloud's first point is a head too)
+            const uint32_t cf = (BATCH && i < b1) ? cloud_of(coff, NC, i) : 0u;
+            const bool first = BATCH && i < b1 && (i == 0 || cf != cloud_of(coff, NC, i - 1));
+            const bool hd = (i < b1) && (i == 0 || skey[i] != skey[i - 1] || first);
             uint32_t before, round;
             cta_rank(hd, s_w, before, round);
             if (hd) { vp.vstart[base + before] = i; vp.vkey[base + before] = skey[i]; }
+            if (first) vp.cvox[cf] = base + before;
             base += round;
         }
     }
@@ -555,8 +628,21 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
         const uint32_t v = v0 + lane;
         if (v >= n_vox) continue;
         float4 c = vox_centroid_of(J.vin, sidx, vp.vstart, v);
-        c = vox_label_of(J.vin, sidx, vp.vstart, vp.vkey, g, n_vox, c);
-        J.vout[v] = J.xform_out ? affine(J.T_out, c) : c;
+        if (!BATCH) {
+            c = vox_label_of(J.vin, sidx, vp.vstart, vp.vkey, g, n_vox, c);
+            J.vout[v] = J.xform_out ? affine(J.T_out, c) : c;
+        } else {
+            // cloud f's voxels are [vo, vo + nvf) of the global list; the label search stays inside them
+            const uint32_t f = cloud_of(coff, NC, vp.vstart[v]);
+            const uint32_t vo = vp.cvox[f], o1 = coff[f + 1];
+            const bool last = v + 1 == n_vox || vp.vstart[v + 1] >= o1;
+            if (J.restore_labels) {
+                const uint32_t nvf = last ? v + 1 - vo : lower_bound_u32(vp.vstart + v + 1, n_vox - v - 1, o1) + v + 1 - vo;
+                c = vox_label_of(J.vin, sidx, vp.vstart + vo, vp.vkey + vo, g + f, nvf, c);
+            }
+            J.vout[coff[f] + (v - vo)] = J.xform_out ? affine(J.T_out, c) : c;
+            if (last) J.cloud_nvox[f] = v + 1 - vo;
+        }
     }
     PH(15);
 #undef PH
@@ -564,32 +650,86 @@ __global__ void __launch_bounds__(FT, 1) k_node_fused(FusedJob J) {
 
 size_t partition_tmp_words(uint32_t n) { return (size_t)(n + PART_CHUNK - 1) / PART_CHUNK + 1; }
 
-size_t voxelize_tmp_bytes(uint32_t n) {
+size_t voxelize_tmp_bytes(uint32_t n, uint32_t n_clouds) {
     const size_t nseg = ((size_t)n + rs_seg_len(n) - 1) / rs_seg_len(n) + 1;
-    // key/idx ping-pong (4 arrays), two digit-histogram matrices + digit totals, head-chunk counters, voxel starts/keys, per-CTA min/max partials
-    return sizeof(uint32_t) * ((size_t)4 * n + 2 * (size_t)RD * nseg + RD + partition_tmp_words(n) + 2 * ((size_t)n + 2) + 64 + 6 * (size_t)kFusedMaxGrid);
+    const size_t nc = n_clouds < 1 ? 1 : n_clouds;
+    // key/idx ping-pong (4 arrays), two digit-histogram matrices + digit totals, head-chunk counters, voxel starts/keys, per-CTA
+    // min/max partials per cloud, first voxel per cloud (batched)
+    return sizeof(uint32_t) * ((size_t)4 * n + 2 * (size_t)RD * nseg + RD + partition_tmp_words(n) + 2 * ((size_t)n + 2) + 64 +
+                               6 * (size_t)kFusedMaxGrid * nc + (n_clouds ? nc : 0));
 }
 
 cudaError_t launch_node_fused(cudaStream_t st, const FusedJob& J, int sm_count, int max_ctas) {
     constexpr size_t SMEM = sizeof(uint32_t) * FW * RD;
-    static int max_ctas_per_sm = -1;
-    if (max_ctas_per_sm < 0) {
-        cudaError_t e = cudaFuncSetAttribute(k_node_fused, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM);
+    const bool batch = J.n_clouds > 0;
+    const void* kern = batch ? (const void*)k_node_fused<true> : (const void*)k_node_fused<false>;
+    static int max_ctas_per_sm[2] = {-1, -1};
+    int& mc = max_ctas_per_sm[batch ? 1 : 0];
+    if (mc < 0) {
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM);
         if (e != cudaSuccess) return e;
         int v = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, k_node_fused, FT, SMEM);
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, kern, FT, SMEM);
         if (e != cudaSuccess) return e;
-        max_ctas_per_sm = v;
+        mc = v;
     }
-    if (max_ctas_per_sm < 1) return cudaErrorLaunchOutOfResources;
-    const uint32_t work = J.vn > J.pn ? J.vn : J.pn;
+    const int max_ctas_per_sm_ = mc;
+    if (max_ctas_per_sm_ < 1) return cudaErrorLaunchOutOfResources;
+    if (batch && (J.has_part || !J.cloud_off || !J.cloud_nvox || !J.d_n_out)) return cudaErrorInvalidValue;
+    const uint32_t work = J.vn > J.pn || batch ? J.vn : J.pn;
     uint32_t G = (work + FT - 1) / FT;
-    const uint32_t cap = (uint32_t)std::min<long long>((long long)sm_count * max_ctas_per_sm, (long long)kFusedMaxGrid);
+    const uint32_t cap = (uint32_t)std::min<long long>((long long)sm_count * max_ctas_per_sm_, (long long)kFusedMaxGrid);
     G = G < 1u ? 1u : (G > cap ? cap : G);
     if (max_ctas > 0 && G > (uint32_t)max_ctas) G = (uint32_t)max_ctas;      // look-ahead jobs leave most SMs to the current node's path
     FusedJob jj = J;
     void* args[] = {&jj};
-    return cudaLaunchCooperativeKernel((const void*)k_node_fused, dim3(G), dim3(FT), args, SMEM, st);
+    return cudaLaunchCooperativeKernel(kern, dim3(G), dim3(FT), args, SMEM, st);
+}
+
+__global__ void k_expand_xyz(const float* __restrict__ in, float4* __restrict__ out, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = make_float4(in[3 * (size_t)i], in[3 * (size_t)i + 1], in[3 * (size_t)i + 2], 0.0f);
+}
+cudaError_t launch_expand_xyz(cudaStream_t st, const float* in, float4* out, uint32_t n) {
+    if (n == 0) return cudaSuccess;
+    k_expand_xyz<<<(n + 255) / 256, 256, 0, st>>>(in, out, n);
+    return cudaGetLastError();
+}
+
+// stable compaction by a keep byte: kept points per chunk, chunk offsets (one CTA), ordered scatter
+__global__ void __launch_bounds__(FT) k_keep_count(const uint8_t* __restrict__ keep, uint32_t n, uint32_t* __restrict__ chunk) {
+    __shared__ uint32_t s_w[FW];
+    const uint32_t b0 = blockIdx.x * PART_CHUNK, b1 = min(n, b0 + PART_CHUNK);
+    uint32_t c = 0;
+    for (uint32_t i = b0 + threadIdx.x; i < b1; i += FT) c += keep[i] ? 1u : 0u;
+    const uint32_t t = cta_sum(c, s_w);
+    if (threadIdx.x == 0) chunk[blockIdx.x] = t;
+}
+__global__ void __launch_bounds__(FT) k_keep_scan(uint32_t* chunk, uint32_t n_chunks, uint32_t* total) {
+    __shared__ uint32_t s_part[34];
+    cta_scan_u32(chunk, n_chunks, total, s_part);
+}
+__global__ void __launch_bounds__(FT) k_keep_scatter(const float4* __restrict__ pts, const uint8_t* __restrict__ keep, uint32_t n,
+                                                     const uint32_t* __restrict__ chunk, float4* __restrict__ out) {
+    __shared__ uint32_t s_w[FW];
+    const uint32_t b0 = blockIdx.x * PART_CHUNK, b1 = min(n, b0 + PART_CHUNK);
+    uint32_t base = chunk[blockIdx.x];
+    for (uint32_t r0 = b0; r0 < b1; r0 += FT) {
+        const uint32_t i = r0 + threadIdx.x;
+        const bool k = i < b1 && keep[i];
+        uint32_t before, round;
+        cta_rank(k, s_w, before, round);
+        if (k) out[base + before] = pts[i];
+        base += round;
+    }
+}
+cudaError_t launch_compact_keep(cudaStream_t st, const float4* pts, const uint8_t* keep, uint32_t n, float4* out, uint32_t* d_n, uint32_t* tmp) {
+    const uint32_t chunks = (n + PART_CHUNK - 1) / PART_CHUNK;
+    if (chunks == 0) return cudaMemsetAsync(d_n, 0, sizeof(uint32_t), st);
+    k_keep_count<<<chunks, FT, 0, st>>>(keep, n, tmp);
+    k_keep_scan<<<1, FT, 0, st>>>(tmp, chunks, d_n);
+    k_keep_scatter<<<chunks, FT, 0, st>>>(pts, keep, n, tmp, out);
+    return cudaGetLastError();
 }
 
 }  // namespace erasor

@@ -39,12 +39,21 @@ struct FusedJob {
     // order; *d_total_sel receives the number selected
     int has_part; PartPred P; Mat4 T_sel; int xform_sel; const float4* pin; uint32_t pn; uint32_t* chunk_tmp /*partition_tmp_words(pn)*/;
     uint32_t* d_total_sel; float4* out_sel; float4* out_rest;
+    // Batched U3 (n_clouds > 0; no U1 job): vin[cloud_off[f] .. cloud_off[f + 1]) for f < n_clouds are independent clouds, each
+    // voxelised on its own grid grid[f] exactly as one call would; cloud f's voxels go to vout[cloud_off[f] ..) in ascending
+    // key, their number to cloud_nvox[f]; *d_n_out receives the total.  cloud_off lives in device memory.  restore_labels = 0
+    // skips the 1-NN label restore (the centroid keeps the averaged fourth component).  n_clouds = 0: the single-cloud job above.
+    uint32_t n_clouds = 0; const uint32_t* cloud_off = nullptr; uint32_t* cloud_nvox = nullptr; int restore_labels = 1;
 };
 size_t partition_tmp_words(uint32_t n);
-size_t voxelize_tmp_bytes(uint32_t n);
+size_t voxelize_tmp_bytes(uint32_t n, uint32_t n_clouds = 1);
 cudaError_t launch_node_fused(cudaStream_t st, const FusedJob& job, int sm_count, int max_ctas = 0 /*0: as many as the job wants, up to one per SM*/);
 
 cudaError_t launch_affine_copy(cudaStream_t st, const Mat4& T, bool do_transform, const float4* in, float4* out, uint32_t n);
+// packed x y z (12 bytes per point) -> float4 with w = 0
+cudaError_t launch_expand_xyz(cudaStream_t st, const float* in, float4* out, uint32_t n);
+// stable compaction: out[0..*d_n) = the points of pts[0..n) whose keep byte is nonzero, in order; tmp: partition_tmp_words(n)
+cudaError_t launch_compact_keep(cudaStream_t st, const float4* pts, const uint8_t* keep, uint32_t n, float4* out, uint32_t* d_n, uint32_t* tmp);
 
 // epilogue of callback_node (OfflineMapUpdater.cpp:281-290) in one launch: up to four copy segments, each optionally through
 // the float affine T (pcl::transformPointCloud)

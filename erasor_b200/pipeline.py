@@ -58,6 +58,75 @@ def run_sequence(nodes, up, ep, voxelize: Optional[mapgen.Voxelizer] = None, mak
     return res
 
 
+class _DeviceNodeMode:
+    """The resident map plus one handle attached to it: the default back end of run_frame_independent."""
+
+    def __init__(self, up, ep, initial_map, device: int = 0):
+        from . import capi
+        self.map = capi.Map(initial_map, device=device)
+        self.h = capi.Handle(ep, device=device)
+        self.h.attach_map(self.map)
+
+    def process_scans(self, poses7, scans, offsets, query_voxel_size, lidar2body, voi_max_range):
+        self.h.process_scans(poses7, scans, offsets, query_voxel_size, lidar2body, voi_max_range=voi_max_range)
+
+    def save_static_map(self, voxel_size: float) -> np.ndarray:
+        return self.h.save_static_map(voxel_size)
+
+    def close(self):
+        self.h.close()
+        self.map.close()
+
+
+def run_frame_independent(nodes: Iterable[Node], initial_map: np.ndarray, up, ep, nodes_per_step: int = 20, device: int = 0,
+                          out_dir: Optional[str] = None, make_handle: Optional[Callable] = None) -> dict:
+    """The frame-independent mode from raw scans: every processed node is tested against the same initial map and the verdicts
+    are ANDed (DESIGN section 7), instead of the sequential updater's map that changes node by node.  A node is processed by
+    the updater's counter rule (call k, 0-based, iff (k + 1) % removal_interval == 0).  Processed nodes go in steps of
+    nodes_per_step through erasor_process_scans (voxelise + lidar -> body on the device), then save_static_map at
+    up.map_voxel_size.  make_handle(up, ep, initial_map) must return an object with process_scans(poses7, scans, offsets,
+    query_voxel_size, lidar2body, voi_max_range), save_static_map(voxel) and close() (default: the device map + handle)."""
+    if make_handle is None:
+        make_handle = lambda u, e, m: _DeviceNodeMode(u, e, m, device=device)
+    initial_map = np.ascontiguousarray(initial_map, dtype=np.float32)
+    h = make_handle(up, ep, initial_map)
+    step = max(1, int(nodes_per_step))
+    seen = processed = 0
+    poses, scans = [], []
+
+    def flush():
+        if not scans:
+            return
+        off = np.cumsum([0] + [len(c) for c in scans]).astype(np.uint64)
+        cat = np.concatenate(scans) if int(off[-1]) else np.zeros((0, 4), dtype=np.float32)
+        h.process_scans(np.stack(poses).astype(np.float64), cat, off, float(up.query_voxel_size), list(up.lidar2body), float(up.max_range))
+        poses.clear()
+        scans.clear()
+
+    try:
+        for seq, odom, cloud in nodes:
+            seen += 1
+            if seen % int(up.removal_interval) != 0:
+                continue
+            processed += 1
+            poses.append(np.asarray(odom, dtype=np.float64).reshape(7))
+            scans.append(np.ascontiguousarray(cloud, dtype=np.float32).reshape(-1, 4))
+            if len(scans) == step:
+                flush()
+        flush()
+        static_map = h.save_static_map(float(up.map_voxel_size))
+    finally:
+        if hasattr(h, "close"):
+            h.close()
+    res = {"static_map": static_map, "nodes": seen, "processed_scans": processed, "naive_map": initial_map,
+           "quality": evaluate.evaluate(initial_map, static_map, voxelsize=0.2)}
+    if out_dir:
+        os.makedirs(out_dir, exist_ok=True)
+        name = getattr(up, "data_name", "seq")
+        evaluate.write_pcd_ascii(os.path.join(out_dir, f"{name}_frame_independent_result.pcd"), static_map)
+    return res
+
+
 def run_semantickitti(dataset_root: str, sequence: str, init_stamp: int, end_stamp: int, interval: int, config_yaml: str,
                       out_dir: Optional[str] = None, **kw) -> dict:
     """SemanticKITTI files + a reference config/*.yaml -> static map and PR/RR."""

@@ -162,6 +162,35 @@ public:
         keep.resize(erasor_map_size(map_));
         return keep;
     }
+    // The same on raw scans in the LiDAR frame: every scan is voxelised at query_voxel_size and moved by lidar2body
+    // (x y z qx qy qz qw) on the device first, as callback_node prepares its query (OfflineMapUpdater.cpp:237-241).
+    std::vector<uint8_t> process_scans(const std::vector<std::array<double, 7>>& poses, const std::vector<PointCloud>& scans, double query_voxel_size,
+                                       const std::array<double, 7>& lidar2body, double voi_max_range = 0.0) {
+        if (!map_) throw std::logic_error("ERASOR: load_global_map first");
+        if (poses.size() != scans.size() || poses.empty()) throw std::invalid_argument("ERASOR: one pose per scan");
+        const size_t F = poses.size();
+        std::vector<uint64_t> so(F + 1, 0);
+        for (size_t f = 0; f < F; ++f) so[f + 1] = so[f] + scans[f].size();
+        PointCloud s(so[F]);
+        for (size_t f = 0; f < F; ++f) std::copy(scans[f].begin(), scans[f].end(), s.begin() + static_cast<std::ptrdiff_t>(so[f]));
+        erasor_scan_params_t sp{};
+        sp.query_voxel_size = query_voxel_size;
+        std::copy(lidar2body.begin(), lidar2body.end(), sp.lidar2body);
+        std::vector<uint8_t> keep(std::max<size_t>(erasor_map_size(map_), 1));
+        check(erasor_process_scans(h_, &sp, poses[0].data(), reinterpret_cast<const float*>(s.data()), so.data(), static_cast<int>(F), voi_max_range,
+                                   nullptr, keep.data(), ERASOR_PTR_HOST));
+        keep.resize(erasor_map_size(map_));
+        return keep;
+    }
+    // save_static_map of the resident map: voxelize_preserving_labels(map[keep], voxel_size) (OfflineMapUpdater.cpp:174-196)
+    PointCloud save_static_map(float voxel_size) {
+        if (!map_) throw std::logic_error("ERASOR: load_global_map first");
+        size_t n = 0;
+        check(erasor_save_static_map(h_, voxel_size, nullptr, 0, &n));
+        PointCloud out(n);
+        if (n) check(erasor_save_static_map(h_, voxel_size, reinterpret_cast<float*>(out.data()), n, &n));
+        return out;
+    }
     void reset_static_mask() { if (map_ && erasor_map_reset_keep(map_) != ERASOR_OK) throw std::runtime_error("ERASOR: erasor_map_reset_keep"); }
     // frame-sharded job: every rank processes its own nodes, then ONE all-gather (bit-packed masks over NVLink) + AND gives
     // every rank the job's static mask.  id128 from erasor_comm_unique_id() on rank 0, shipped by the host program.

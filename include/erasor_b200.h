@@ -207,8 +207,35 @@ int erasor_process_nodes(erasor_handle_t h, const double* poses7, const float* q
                          double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind);
 int erasor_process_nodes_async(erasor_handle_t h, const double* poses7, const float* query_xyzi, const uint64_t* query_offsets, int n_frames,
                                double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind);
-/* per-node counters of the last erasor_process_nodes: points inside the VoI (|map_voi_|), flagged bins, rejected points */
+/* per-node counters of the last erasor_process_nodes / erasor_process_scans: points inside the VoI (|map_voi_|), flagged
+ * bins, rejected points */
 int erasor_get_node_stats(erasor_handle_t h, uint32_t* n_voi_points, uint32_t* n_flagged_bins, uint32_t* n_rejected_points);
+
+/* Node mode on raw scans.  What callback_node does to a scan before ERASOR::set_inputs (OfflineMapUpdater.cpp:237-241),
+ * on the device and for the whole batch in one launch: query_f = transform(voxelize_preserving_labels(scan_f,
+ * query_voxel_size), lidar2body), each scan on its own pcl::VoxelGrid (a scan whose grid overflows int32 passes unfiltered,
+ * an empty scan gives an empty query).  Then exactly erasor_process_nodes on those queries: same outputs, same counters.
+ *   scans[scan_offsets[f] .. scan_offsets[f+1]): scan f in the LiDAR frame, x y z i (16 bytes per point), or packed x y z
+ *   (12 bytes) with ERASOR_PTR_QUERY_XYZ in ptr_kind.  The masks never read a query's intensity, so labels are not restored.
+ * The step needs no device -> host read-back of the voxel counts: the host cuts the query work from the raw scan sizes,
+ * the device clamps it to the counts.  Invalid voxel size, poses or offsets: ERASOR_E_INVALID. */
+typedef struct {
+    double query_voxel_size;       /* /erasor/query_voxel_size (> 0) */
+    double lidar2body[7];          /* /tf/lidar2body: x y z qx qy qz qw */
+} erasor_scan_params_t;
+int erasor_process_scans(erasor_handle_t h, const erasor_scan_params_t* sp, const double* poses7, const float* scans,
+                         const uint64_t* scan_offsets, int n_frames, double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out, int ptr_kind);
+int erasor_process_scans_async(erasor_handle_t h, const erasor_scan_params_t* sp, const double* poses7, const float* scans,
+                               const uint64_t* scan_offsets, int n_frames, double voi_max_range, uint8_t* frame_keep, uint8_t* keep_out,
+                               int ptr_kind);
+/* The voxelised body-frame queries of the last erasor_process_scans submission (its last sub-batch when the batch was split),
+ * x y z per point (HOST, 3 floats each), frame after frame, each in voxel-key order; offsets[0 .. n + 1) receives the
+ * per-frame starts (n = frames of that submission; HOST, n + 1 entries).  xyz == NULL: offsets only.  Synchronous. */
+int erasor_get_scan_queries(erasor_handle_t h, float* xyz, size_t cap, uint64_t* offsets);
+/* OfflineMapUpdater::save_static_map for the attached map (OfflineMapUpdater.cpp:174-196, no file): voxelize_preserving_labels
+ * of the map points whose keep byte is 1, in map order, at voxel_size, labels restored (HOST out_xyzi, x y z i).  *n receives
+ * the size; out_xyzi == NULL (or cap < *n with ERASOR_E_CAPACITY) is the size query.  Synchronous. */
+int erasor_save_static_map(erasor_handle_t h, float voxel_size, float* out_xyzi, size_t cap, size_t* n);
 
 /* ---- the path's single collective, behind the C ABI (north_star: one NCCL all-gather of the static masks) ------------ */
 /* A communicator owned by the handle (NCCL is loaded with dlopen("libnccl.so.2") on first use).  Rank 0 calls
