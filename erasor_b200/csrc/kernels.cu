@@ -958,7 +958,7 @@ static void k2_smem_plan(int B, bool with_complement, uint32_t& SW, size_t& smem
     const uint32_t n_slots_max = with_complement ? (uint32_t)B + 1u : (uint32_t)B;
     const size_t full = sizeof(uint32_t) * (size_t)(W + 1) * n_slots_max + fixed;
     const size_t two_per_sm = 111 * 1024;                 // two CTAs per SM: (227 KB - static shared memory) / 2
-    const size_t budget = full <= two_per_sm ? full : two_per_sm;      // 40 x 360: 2304-slot windows (config 5 flags ~2060 bins per frame)
+    const size_t budget = full <= two_per_sm ? full : two_per_sm;      // 40 x 360: 2356-slot windows (config 5 flags ~2060 bins per frame)
     SW   = (uint32_t)std::min<size_t>(std::max<uint32_t>(n_slots_max, 1u), std::max<size_t>(1, (budget - fixed) / (sizeof(uint32_t) * (W + 1))));
     smem = sizeof(uint32_t) * (size_t)(W + 1) * SW + fixed;
 }
